@@ -22,6 +22,14 @@ def _have_gpu():
 
 
 def pytest_collection_modifyitems(config, items):
+    import reference_runs
+    if reference_runs.RECORDING:
+        # only the comparisons with the reference run; on a machine without a device the GPU-marked ones skip after
+        # their reference side has been recorded (fixture `reference`)
+        keep = [it for it in items if "reference" in getattr(it, "fixturenames", ())]
+        config.hook.pytest_deselected(items=[it for it in items if it not in keep])
+        items[:] = keep
+        return
     # GPU tests are selected with `-m gpu` on the GPU box; if they get collected on a machine
     # without a device (plain `pytest tests/`), skip rather than fail.
     if _have_gpu():
@@ -52,6 +60,31 @@ def reflib(built):
     if not os.path.exists(ob.REF_SO):
         pytest.skip("oracle/_ref/libnlopt_ref.so not built (needs /root/reference at build time)")
     return Library(ob.REF_SO, extensions=False)
+
+
+@pytest.fixture(scope="session")
+def _reference_store(built):
+    import reference_runs
+    lib = None
+    if reference_runs.RECORDING:
+        import oracle_bindings as ob
+        from nlopt_b200 import Library
+        lib = Library(ob.REF_SO, extensions=False)
+    store = reference_runs.Store(lib)
+    yield store
+    store.save()
+
+
+@pytest.fixture
+def reference(request, _reference_store):
+    """reference(key, compute) -> the unmodified reference's result of one run, stored under tests/golden
+    (tests/reference_runs.py); compute(lib) produces it from the reference library when the results are regenerated."""
+    def get(key, compute):
+        result = _reference_store.get(key, compute)
+        if _reference_store.lib is not None and request.node.get_closest_marker("gpu") and not _have_gpu():
+            pytest.skip("reference side recorded; the comparison needs a CUDA device")
+        return result
+    return get
 
 
 @pytest.fixture(scope="session")

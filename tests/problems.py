@@ -45,7 +45,9 @@ def lin_constraint(k, n):
     def c(x, grad):
         if grad.size > 0:
             grad[:] = w
-        return float(np.dot(w, x)) - b
+        # numpy's pairwise sum, not np.dot: BLAS splits a long dot product over its threads, so its last bits depend on
+        # the host's core count, and the stored reference results are compared bit for bit
+        return float(np.sum(w * x)) - b
     return c
 
 

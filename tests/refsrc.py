@@ -1,91 +1,43 @@
-"""Helpers that use the reference tree IN PLACE (this container only; never copied into the repo):
-generate nlopt.hpp the way cmake/generate-cpp.cmake does and compile the reference's own C++ tests
-against a library of ours.  Everything is skipped when /root/reference is absent (GPU box)."""
+"""The reference's own test programs against a library of ours.  build() compiles them, unmodified, into
+oracle/_ref/refprog (`make refprog`, oracle/Makefile); here their objects are linked against a given library exporting
+the NLopt C ABI.  The reference tree itself is only needed by test/t_python.py, a script that is run in place."""
 import os
-import re
 import subprocess
 
 REF = os.environ.get("NLOPT_REFERENCE_DIR", "/root/reference")
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+PROG = os.path.join(ROOT, "oracle", "_ref", "refprog")
+NOT_BUILT = "oracle/_ref/refprog not built (make -C oracle refprog needs the reference's sources at build time)"
 
 
 def available():
-    return os.path.isfile(os.path.join(REF, "src", "api", "nlopt-in.hpp"))
+    return os.path.isfile(os.path.join(REF, "test", "t_python.py"))
 
 
-def generate_hpp(outdir):
-    """nlopt-in.hpp + the enum block derived from nlopt.h (cmake/generate-cpp.cmake:39-52)."""
-    os.makedirs(outdir, exist_ok=True)
-    src = open(os.path.join(REF, "src", "api", "nlopt-in.hpp")).read().splitlines()
-    hdr = open(os.path.join(REF, "src", "api", "nlopt.h")).read().splitlines()
-    out = []
-    for line in src:
-        out.append(line)
-        if "GEN_ENUMS_HERE" in line:
-            out.append("  enum algorithm {")
-            for h in hdr:
-                if re.search(r"    NLOPT_[A-Z0-9_]+", h):
-                    out.append(h.replace("NLOPT_", ""))
-                    if "NLOPT_NUM_ALGORITHMS" in h:
-                        out += ["  };", "  enum result {"]
-                    elif "NLOPT_NUM_RESULTS" in h:
-                        out.append("  };")
-    path = os.path.join(outdir, "nlopt.hpp")
-    open(path, "w").write("\n".join(out) + "\n")
-    return path
+def built():
+    return all(os.path.exists(os.path.join(PROG, f)) for f in
+               ("t_tutorial_refhdr.o", "t_tutorial_ourhdr.o", "cpp_functor_refhdr.o", "testopt.o", "testfuncs.o", "timer.o",
+                "mt19937ar.o"))
 
 
-def compile_reference_test(name, libpath, outdir, use_our_header):
-    """g++ <ref>/test/<name> against `libpath`; returns the executable path."""
-    generate_hpp(outdir)
-    exe = os.path.join(outdir, os.path.splitext(name)[0] + ("_ourhdr" if use_our_header else "_refhdr"))
-    inc = os.path.join(ROOT, "include") if use_our_header else os.path.join(REF, "src", "api")
+def _link(compiler, objs, libpath, exe, extra=()):
     libdir, libfile = os.path.split(libpath)
-    cmd = ["g++", "-O1", "-std=c++11", f"-I{outdir}", f"-I{inc}", os.path.join(REF, "test", name), "-o", exe,
-           f"-L{libdir}", f"-l:{libfile}", f"-Wl,-rpath,{libdir}"]
-    subprocess.check_call(cmd)
+    subprocess.check_call([compiler, *[os.path.join(PROG, o) for o in objs], "-o", exe, f"-L{libdir}", f"-l:{libfile}",
+                           f"-Wl,-rpath,{libdir}", *extra])
     return exe
 
 
-def compile_reference_testopt(libpath, outdir):
-    """The reference's benchmark driver test/testopt.c (+ testfuncs.c and, as test/CMakeLists.txt:26 does, the two
-    util sources whose symbols it uses directly) compiled unmodified against `libpath`."""
+def reference_test(name, libpath, outdir, use_our_header):
+    """test/<name>.cxx compiled over the reference-generated nlopt.hpp and the reference's nlopt.h (or ours, include/),
+    linked against `libpath`; returns the executable path."""
     os.makedirs(outdir, exist_ok=True)
-    libdir, libfile = os.path.split(libpath)
-    exe = os.path.join(outdir, "testopt_" + os.path.splitext(libfile)[0])
-    cmd = ["gcc", "-O1", "-DHAVE_GETOPT", "-DHAVE_GETOPT_H", f"-I{REF}/src/api", f"-I{REF}/src/util",
-           f"-I{os.path.join(ROOT, 'oracle', 'ref_config')}", os.path.join(REF, "test", "testopt.c"),
-           os.path.join(REF, "test", "testfuncs.c"), os.path.join(REF, "src", "util", "timer.c"),
-           os.path.join(REF, "src", "util", "mt19937ar.c"), "-o", exe, f"-L{libdir}", f"-l:{libfile}", f"-Wl,-rpath,{libdir}", "-lm"]
-    subprocess.check_call(cmd)
-    return exe
+    hdr = "ourhdr" if use_our_header else "refhdr"
+    return _link("g++", [f"{name}_{hdr}.o"], libpath, os.path.join(outdir, f"{name}_{hdr}"))
 
 
-REFPROG_DIR = os.path.join(ROOT, "tests", "_build", "refprog")
-
-
-def build_reference_programs_for_gpu():
-    """The reference's own test programs -- test/t_tutorial.cxx and test/cpp_functor.cxx over the reference-generated
-    nlopt.hpp, and the benchmark driver test/testopt.c -- compiled UNMODIFIED, where the sources lie, with `-lnlopt`
-    against this repository's libnlopt.so.1 (nlopt_b200/compat).  Outputs go to tests/_build/refprog (git-ignored; it
-    travels to the GPU box with the snapshot, where tests/test_dropin_gpu.py runs them on the CUDA library).  The
-    run-time search path is relative ($ORIGIN), so the binaries work from any checkout location."""
-    if not available():
-        return []
-    compat = os.path.join(ROOT, "nlopt_b200", "compat")
-    os.makedirs(REFPROG_DIR, exist_ok=True)
-    generate_hpp(REFPROG_DIR)
-    rpath = "-Wl,-rpath,$ORIGIN/../../../nlopt_b200/compat"
-    out = []
-    for name in ("t_tutorial.cxx", "cpp_functor.cxx"):
-        exe = os.path.join(REFPROG_DIR, os.path.splitext(name)[0])
-        subprocess.check_call(["g++", "-O1", "-std=c++11", f"-I{REFPROG_DIR}", f"-I{os.path.join(REF, 'src', 'api')}",
-                               os.path.join(REF, "test", name), "-o", exe, f"-L{compat}", "-lnlopt", rpath])
-        out.append(exe)
-    exe = os.path.join(REFPROG_DIR, "testopt")
-    subprocess.check_call(["gcc", "-O1", "-DHAVE_GETOPT", "-DHAVE_GETOPT_H", f"-I{REF}/src/api", f"-I{REF}/src/util",
-                           f"-I{os.path.join(ROOT, 'oracle', 'ref_config')}", os.path.join(REF, "test", "testopt.c"),
-                           os.path.join(REF, "test", "testfuncs.c"), os.path.join(REF, "src", "util", "timer.c"),
-                           os.path.join(REF, "src", "util", "mt19937ar.c"), "-o", exe, f"-L{compat}", "-lnlopt", rpath, "-lm"])
-    out.append(exe)
-    return out
+def reference_testopt(libpath, outdir):
+    """The reference's benchmark driver test/testopt.c (+ testfuncs.c and, as test/CMakeLists.txt:26 does, the two util
+    sources whose symbols it uses directly) linked against `libpath`."""
+    os.makedirs(outdir, exist_ok=True)
+    exe = os.path.join(outdir, "testopt_" + os.path.splitext(os.path.basename(libpath))[0])
+    return _link("gcc", ["testopt.o", "testfuncs.o", "timer.o", "mt19937ar.o"], libpath, exe, ["-lm"])

@@ -106,9 +106,14 @@ def _call(lib, c):
                 mineq=c.get("mineq"), **c["kw"])
 
 
+def _ref_call(reference, key, c):
+    return reference(key, lambda lib: {k: v for k, v in _call(lib, c).items() if k != "opt"})
+
+
 @pytest.mark.parametrize("name,case", _cases(), ids=[n for n, _ in _cases()])
-def test_auglag_host_logic_matches_reference(hosttest_lib, reflib, name, case):
-    a, b = _call(hosttest_lib, case), _call(reflib, case)
+def test_auglag_host_logic_matches_reference(hosttest_lib, reference, name, case):
+    b = _ref_call(reference, f"auglag/{name}", case)
+    a = _call(hosttest_lib, case)
     assert b["ret"] > 0
     if _sub_has_constraints(case):
         # the sub-problems are constrained MMA runs: rounding-level differences of the dual sums are amplified by
@@ -138,10 +143,11 @@ def test_auglag_argument_checks(hosttest_lib):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("name,case", _cases(), ids=[n for n, _ in _cases()])
-def test_auglag_on_gpu_matches_reference(built, reflib, name, case):
+def test_auglag_on_gpu_matches_reference(built, reference, name, case):
     """Same runs through the product library: the augmented-Lagrangian objective and its gradient are assembled on
     the device (penalty rows uploaded, penalty_axpy_kernel); MMA/CCSAQ run on the GPU."""
-    a, b = _call(None, case), _call(reflib, case)
+    b = _ref_call(reference, f"auglag/{name}", case)
+    a = _call(None, case)
     assert a["ret"] > 0 and b["ret"] > 0
     penalty_only_mma = not _sub_has_constraints(case) and case.get("local", (None,))[0] != nl.LD_CCSAQ
     if case["kw"].get("maxeval") == 57:          # short fixed-length run: same count, same point to rounding
@@ -161,18 +167,19 @@ def test_auglag_on_gpu_matches_reference(built, reflib, name, case):
 
 
 @pytest.mark.gpu
-def test_auglag_large_n_gradient_assembly(built, reflib):
+def test_auglag_large_n_gradient_assembly(built, reference):
     """n large enough to exercise the sharded upload + axpy path; short fixed run against the reference."""
     n = 20011
     c = dict(alg=nl.LD_AUGLAG, n=n, f=lin_obj, ineq=[(halfspace, 1e-8)], eq=[(circle_eq, 1e-8), (plane_eq, 1e-8)],
              lb=np.full(n, -2.0), ub=np.full(n, 2.0), x0=np.full(n, 0.01), kw=dict(xtol_rel=1e-10, maxeval=40))
-    a, b = _call(None, c), _call(reflib, c)
+    b = _ref_call(reference, "auglag/large_n", c)
+    a = _call(None, c)
     assert a["ret"] == b["ret"] and a["numevals"] == b["numevals"]
     assert abs(a["minf"] - b["minf"]) <= 1e-7 * max(1.0, abs(b["minf"]))
     assert np.max(np.abs(a["x"] - b["x"])) <= 1e-6
 
 
-def test_auglag_maximize_stopval_and_forced_stop(hosttest_lib, reflib):
+def test_auglag_maximize_stopval_and_forced_stop(hosttest_lib, reference):
     """Option surface around the outer loop: maximisation (sign flip, optimize.c:1014-1024), stopval on a feasible
     point (auglag.c:272), nlopt_force_stop from inside a callback (auglag.c:39, :218) -- same outcome as the reference."""
     n = 12
@@ -184,30 +191,31 @@ def test_auglag_maximize_stopval_and_forced_stop(hosttest_lib, reflib):
             grad[:] = -grad
         return -v
 
-    res = {}
-    for name, lib in (("ours", hosttest_lib), ("ref", reflib)):
+    def maximize(lib):
         o = nl.opt(nl.LD_AUGLAG, n, library=lib)
         o.set_lower_bounds(lb); o.set_upper_bounds(ub)
         o.set_max_objective(neg_obj)
         o.add_equality_constraint(circle_eq, 1e-8)
         o.set_xtol_rel(1e-6); o.set_maxeval(2000)
         x = o.optimize(x0.copy())
-        res[name] = (o.last_optimize_result(), o.get_numevals(), o.last_optimum_value(), x)
+        return o.last_optimize_result(), o.get_numevals(), o.last_optimum_value(), x
+    res = {"ref": reference("auglag/maximize", maximize), "ours": maximize(hosttest_lib)}
     assert res["ours"][0] == res["ref"][0] and res["ours"][1] == res["ref"][1]
     assert abs(res["ours"][2] - res["ref"][2]) <= 1e-9 and np.max(np.abs(res["ours"][3] - res["ref"][3])) <= 1e-7
 
-    for name, lib in (("ours", hosttest_lib), ("ref", reflib)):
+    def stopval(lib):
         o = nl.opt(nl.LD_AUGLAG, n, library=lib)
         o.set_lower_bounds(lb); o.set_upper_bounds(ub)
         o.set_min_objective(lin_obj)
         o.add_inequality_constraint(halfspace, 1e-8)
         o.set_stopval(1.0); o.set_xtol_rel(1e-9); o.set_maxeval(2000)      # any feasible point with f < 1 ends the run
         x = o.optimize(x0.copy())
-        res[name] = (o.last_optimize_result(), o.get_numevals(), o.last_optimum_value(), x)
+        return o.last_optimize_result(), o.get_numevals(), o.last_optimum_value(), x
+    res = {"ref": reference("auglag/stopval", stopval), "ours": stopval(hosttest_lib)}
     assert res["ours"][0] == res["ref"][0] == nl.STOPVAL_REACHED and res["ours"][1] == res["ref"][1]
     assert abs(res["ours"][2] - res["ref"][2]) <= 1e-9
 
-    for name, lib in (("ours", hosttest_lib), ("ref", reflib)):
+    def forced_stop(lib):
         o = nl.opt(nl.LD_AUGLAG, n, library=lib)
         calls = [0]
 
@@ -225,5 +233,6 @@ def test_auglag_maximize_stopval_and_forced_stop(hosttest_lib, reflib):
             o.optimize(x0.copy())
         except Exception:
             pass
-        res[name] = (o.last_optimize_result(), calls[0])
+        return o.last_optimize_result(), calls[0]
+    res = {"ref": reference("auglag/forced_stop", forced_stop), "ours": forced_stop(hosttest_lib)}
     assert res["ours"] == res["ref"] and res["ours"][0] == nl.FORCED_STOP

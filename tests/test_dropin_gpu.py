@@ -52,13 +52,13 @@ def test_user_programs_run_on_the_cuda_library(built, kind, alg):
 
 
 # ---- the reference's own test programs on the CUDA library -------------------------------------------------------
-REFPROG = os.path.join(ROOT, "tests", "_build", "refprog")
+REFPROG = os.path.join(ROOT, "oracle", "_ref", "refprog")
 
 
 def _refprog(name):
     exe = os.path.join(REFPROG, name)
     if not os.path.exists(exe):
-        pytest.skip("tests/_build/refprog not built (needs /root/reference at build time: python __graft_entry__.py)")
+        pytest.skip("oracle/_ref/refprog not built (make -C oracle refprog needs the reference's sources at build time)")
     return exe
 
 

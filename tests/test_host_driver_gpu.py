@@ -1,8 +1,8 @@
 """The comparisons of tests/test_host_driver.py -- every MMA/CCSAQ parameter of optimize.c:798-826, the dual
 tolerances supplied by a local optimiser, infeasible starts, NaN constraints, vector constraints, maximisation,
 stopping rules, threads -- run through the PRODUCT library (CUDA kernels, fused dual solve) instead of the
-CPU-backed build of the host logic.  Same assertions, same tolerances; the unmodified reference (oracle/_ref, which
-travels to the GPU box) is the other side of each comparison."""
+CPU-backed build of the host logic.  Same assertions, same tolerances; the unmodified reference's stored results
+(tests/reference_runs.py) are the other side of each comparison."""
 import numpy as np
 import pytest
 
@@ -21,21 +21,21 @@ def gpulib(built):
 
 
 @pytest.mark.parametrize("alg", [nl.LD_MMA, nl.LD_CCSAQ])
-def test_rosenbrock_vs_reference(gpulib, reflib, alg):
-    H.test_rosenbrock_vs_reference(gpulib, reflib, alg)
+def test_rosenbrock_vs_reference(gpulib, reference, alg):
+    H.test_rosenbrock_vs_reference(gpulib, reference, alg)
 
 
 @pytest.mark.parametrize("alg", [nl.LD_MMA, nl.LD_CCSAQ])
 @pytest.mark.parametrize("opts", [dict(), dict(inner_gradients=0), dict(always_improve=0), dict(sigma_min=0.05),
                                   dict(inner_maxeval=2), dict(rho_init=10.0)])
-def test_algorithm_parameters_vs_reference(gpulib, reflib, alg, opts):
-    H.test_algorithm_parameters_vs_reference(gpulib, reflib, alg, opts)
+def test_algorithm_parameters_vs_reference(gpulib, reference, alg, opts):
+    H.test_algorithm_parameters_vs_reference(gpulib, reference, alg, opts)
 
 
 @pytest.mark.parametrize("alg", [nl.LD_MMA, nl.LD_CCSAQ])
 @pytest.mark.parametrize("opts", [dict(dual_ftol_rel=1e-6), dict(dual_xtol_rel=1e-6), dict(dual_maxeval=5),
                                   dict(dual_ftol_abs=1e-10), dict(dual_xtol_abs=1e-9, dual_ftol_rel=0.0)])
-def test_dual_tolerances_vs_reference(gpulib, reflib, alg, opts):
+def test_dual_tolerances_vs_reference(gpulib, reference, alg, opts):
     """dual_* parameters (optimize.c:822-826) through the persistent solve kernel against the reference over the first 20
     evaluations.  Tolerance: a dual solve that stops on a loose rule stops at a y that depends on the last bits of the
     n-term sums (tree order here, sequential in the reference), so the two runs separate by ~1e-7 relative in f and
@@ -44,24 +44,25 @@ def test_dual_tolerances_vs_reference(gpulib, reflib, alg, opts):
     f, c = H.P.quad_problem(n)
     lb, ub = np.full(n, -1.0), np.full(n, 1.0)
     kw = dict(xtol_rel=1e-7, **opts)
+    b = reference(f"host_driver_gpu/dual_tolerances/{alg}/{H.okey(opts)}",
+                  lambda lib: H.plain(H.run(lib, alg, n, f, [c], [0.0], lb, ub, np.full(n, -0.5), maxeval=20, **kw)))
     a = H.run(gpulib, alg, n, f, [c], [0.0], lb, ub, np.full(n, -0.5), maxeval=20, **kw)
-    b = H.run(reflib, alg, n, f, [c], [0.0], lb, ub, np.full(n, -0.5), maxeval=20, **kw)
     assert a["ret"] == b["ret"] and a["numevals"] == b["numevals"]
     assert abs(a["minf"] - b["minf"]) <= 1e-6 * max(1.0, abs(b["minf"]))
     assert np.max(np.abs(a["x"] - b["x"])) <= 1e-4
 
 
 @pytest.mark.parametrize("alg", [nl.LD_MMA, nl.LD_CCSAQ])
-def test_default_dual_tolerance_agrees_loosely(gpulib, reflib, alg):
-    H.test_default_dual_tolerance_agrees_loosely(gpulib, reflib, alg)
+def test_default_dual_tolerance_agrees_loosely(gpulib, reference, alg):
+    H.test_default_dual_tolerance_agrees_loosely(gpulib, reference, alg)
 
 
-def test_infeasible_start_uses_capped_multipliers(gpulib, reflib):
-    H.test_infeasible_start_uses_capped_multipliers(gpulib, reflib)
+def test_infeasible_start_uses_capped_multipliers(gpulib, reference):
+    H.test_infeasible_start_uses_capped_multipliers(gpulib, reference)
 
 
-def test_unconstrained_m0(gpulib, reflib):
-    H.test_unconstrained_m0(gpulib, reflib)
+def test_unconstrained_m0(gpulib, reference):
+    H.test_unconstrained_m0(gpulib, reference)
 
 
 def test_vector_constraint_equals_scalar_constraints(gpulib):
@@ -76,16 +77,16 @@ def test_stopping_and_forced_stop(gpulib):
     H.test_stopping_and_forced_stop(gpulib)
 
 
-def test_nan_constraint_is_ignored_by_mma(gpulib, reflib):
-    H.test_nan_constraint_is_ignored_by_mma(gpulib, reflib)
+def test_nan_constraint_is_ignored_by_mma(gpulib, reference):
+    H.test_nan_constraint_is_ignored_by_mma(gpulib, reference)
 
 
-def test_local_optimizer_supplies_dual_tolerances(gpulib, reflib):
-    H.test_local_optimizer_supplies_dual_tolerances(gpulib, reflib)
+def test_local_optimizer_supplies_dual_tolerances(gpulib, reference):
+    H.test_local_optimizer_supplies_dual_tolerances(gpulib, reference)
 
 
-def test_deprecated_one_call_api_matches_reference(gpulib, reflib):
-    H.test_deprecated_one_call_api_matches_reference(gpulib, reflib)
+def test_deprecated_one_call_api_matches_reference(gpulib, reference):
+    H.test_deprecated_one_call_api_matches_reference(gpulib, reference)
 
 
 def test_distinct_objects_on_distinct_threads(gpulib):
@@ -110,5 +111,5 @@ def test_maxtime_returns_maxtime(gpulib):
 
 
 @pytest.mark.parametrize("with_constraint_pre", [False, True])
-def test_preconditioned_ccsaq_converges_to_the_reference_optimum(gpulib, reflib, with_constraint_pre):
-    H.test_preconditioned_ccsaq_converges_to_the_reference_optimum(gpulib, reflib, with_constraint_pre)
+def test_preconditioned_ccsaq_converges_to_the_reference_optimum(gpulib, reference, with_constraint_pre):
+    H.test_preconditioned_ccsaq_converges_to_the_reference_optimum(gpulib, reference, with_constraint_pre)

@@ -97,9 +97,10 @@ def _neg(f, x, g):
 
 
 @pytest.mark.parametrize("seed", range(48))
-def test_random_small_problems_match_reference(hosttest_lib, reflib, seed):
+def test_random_small_problems_match_reference(hosttest_lib, reference, seed):
     p = make_problem(1000 + seed)
-    a, b = run(hosttest_lib, p), run(reflib, p)
+    b = reference(f"host_fuzz/small/{1000 + seed}", lambda lib: run(lib, p))
+    a = run(hosttest_lib, p)
     assert a[0] == b[0] and a[1] == b[1], (a[:3], b[:3])
     assert abs(a[2] - b[2]) <= 1e-6 * max(1.0, abs(b[2])), (a[2], b[2])
     assert np.max(np.abs(a[3] - b[3])) <= 1e-5
@@ -107,12 +108,12 @@ def test_random_small_problems_match_reference(hosttest_lib, reflib, seed):
 
 @pytest.mark.parametrize("seed", range(16))
 @pytest.mark.parametrize("stop", ["xtol_rel", "ftol_rel", "xtol_abs"])
-def test_random_small_problems_converge_to_the_reference_optimum(hosttest_lib, reflib, seed, stop):
+def test_random_small_problems_converge_to_the_reference_optimum(hosttest_lib, reference, seed, stop):
     """The same generator run to convergence under each stopping rule (stop.c:81-108): the result class must be a
     success in both libraries and the optimum must agree (which rule fires first may legitimately differ at ties)."""
     p = make_problem(5000 + seed)
-    out = []
-    for lib in (hosttest_lib, reflib):
+
+    def solve(lib):
         o = nl.opt(p["alg"], p["n"], library=lib)
         o.set_lower_bounds(p["lb"]); o.set_upper_bounds(p["ub"])
         o.set_min_objective(p["f"])
@@ -127,9 +128,10 @@ def test_random_small_problems_converge_to_the_reference_optimum(hosttest_lib, r
         else:
             o.set_xtol_abs(np.full(p["n"], 1e-9))
         o.set_maxeval(4000)
-        x = o.optimize(p["x0"].copy())
-        out.append((o.last_optimize_result(), o.last_optimum_value(), x))
-    (ra, fa, xa), (rb, fb, xb) = out
+        o.optimize(p["x0"].copy())
+        return o.last_optimize_result(), o.last_optimum_value()
+    rb, fb = reference(f"host_fuzz/converge/{5000 + seed}/{stop}", solve)
+    ra, fa = solve(hosttest_lib)
     assert ra > 0 and rb > 0
     if ra != nl.MAXEVAL_REACHED and rb != nl.MAXEVAL_REACHED:
         assert abs(fa - fb) <= 1e-5 * max(1.0, abs(fb)), (ra, rb, fa, fb)       # slow CCSAQ tails stop a few 1e-6 apart
@@ -137,13 +139,13 @@ def test_random_small_problems_converge_to_the_reference_optimum(hosttest_lib, r
 
 @pytest.mark.parametrize("alg", [nl.LD_MMA, nl.LD_CCSAQ])
 @pytest.mark.parametrize("poison", ["nan_objective_once", "inf_objective_region", "nan_constraint_late"])
-def test_non_finite_callback_values_are_handled_like_the_reference(hosttest_lib, reflib, alg, poison):
+def test_non_finite_callback_values_are_handled_like_the_reference(hosttest_lib, reference, alg, poison):
     """Comparisons against NaN / inf decide acceptance and conservativeness (mma.c:302-392); whatever the reference
     does with a non-finite callback value, the host logic must do the same (same code, evaluations and point)."""
     n = 6
     lb, ub, x0 = np.full(n, -2.0), np.full(n, 2.0), np.full(n, 0.7)
-    out = []
-    for lib in (hosttest_lib, reflib):
+
+    def solve(lib):
         calls = [0]
 
         def f(x, grad, calls=calls):
@@ -176,8 +178,9 @@ def test_non_finite_callback_values_are_handled_like_the_reference(hosttest_lib,
             x = o.optimize(x0.copy())
         except Exception:
             x = np.full(n, np.nan)
-        out.append((o.last_optimize_result(), o.get_numevals(), o.last_optimum_value(), x))
-    a, b = out
+        return o.last_optimize_result(), o.get_numevals(), o.last_optimum_value(), x
+    b = reference(f"host_fuzz/non_finite/{alg}/{poison}", solve)
+    a = solve(hosttest_lib)
     assert a[0] == b[0] and abs(a[1] - b[1]) <= 1, (a[:3], b[:3])      # the xtol test at f* = 0 may fire one iteration apart
     assert (np.isnan(a[2]) and np.isnan(b[2])) or a[2] == b[2] or abs(a[2] - b[2]) <= 1e-7 * max(1.0, abs(b[2]))
     assert np.allclose(a[3], b[3], atol=1e-6, equal_nan=True)
@@ -185,10 +188,11 @@ def test_non_finite_callback_values_are_handled_like_the_reference(hosttest_lib,
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("seed", range(48))
-def test_random_small_problems_on_gpu_match_reference(built, reflib, seed):
+def test_random_small_problems_on_gpu_match_reference(built, reference, seed):
     """The fixed-seed generator above through the product library (CUDA path)."""
     p = make_problem(1000 + seed)
-    a, b = run(None, p), run(reflib, p)
+    b = reference(f"host_fuzz/small/{1000 + seed}", lambda lib: run(lib, p))
+    a = run(None, p)
     assert a[0] == b[0] and a[1] == b[1], (a[:3], b[:3])
     assert abs(a[2] - b[2]) <= 1e-6 * max(1.0, abs(b[2])), (a[2], b[2])
     assert np.max(np.abs(a[3] - b[3])) <= 1e-5

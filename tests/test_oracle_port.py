@@ -1,6 +1,8 @@
 """The oracle is pinned here: the plain-C port (oracle/ccsa_port.c) against
  (a) the known-answer vectors measured from the reference build (SURVEY.md Appendix B), and
- (b) the unmodified reference itself, compiled into oracle/_ref -- bit for bit."""
+ (b) the unmodified reference itself, compiled into oracle/_ref -- bit for bit (its results are stored in
+     tests/golden/reference_runs.npz, tests/reference_runs.py; arrays as a SHA-256 of their bits)."""
+import hashlib
 import os
 
 import numpy as np
@@ -36,33 +38,41 @@ def test_known_answer_dual(built, variant):
     assert list(r["grad"]) == [-v for v in e["gc"]]
 
 
+def _sha256(x):
+    """digest of an array's bits; every NaN counts as the same NaN and -0.0 as 0.0, as np.array_equal(equal_nan=True) does"""
+    x = np.asarray(x, dtype=np.float64)
+    return hashlib.sha256(np.where(np.isnan(x), np.nan, x + 0.0).tobytes()).hexdigest()
+
+
+def _digest(r):
+    return dict(ret=r["ret"], g0=r["g0"], w=r["w"], gc=r["gc"], xcur_sha256=_sha256(r["xcur"]))
+
+
 def _same(a, b):
     for k in ("ret", "g0", "w"):
         assert a[k] == b[k] or (np.isnan(a[k]) and np.isnan(b[k])), k
     assert np.array_equal(a["gc"], b["gc"], equal_nan=True)
-    assert np.array_equal(a["xcur"], b["xcur"], equal_nan=True)
+    assert a["xcur_sha256"] == b["xcur_sha256"]
 
 
 @pytest.mark.parametrize("n,m", [(1, 0), (2, 2), (7, 1), (1000, 1), (4097, 3), (100000, 4), (20000, 16)])
 @pytest.mark.parametrize("variant", [ob.MMA, ob.CCSAQ])
-def test_port_dual_bitwise_vs_reference(built, variant, n, m):
-    if not ob.ref_dual_available():
-        pytest.skip("oracle/_ref not built")
+def test_port_dual_bitwise_vs_reference(built, reference, variant, n, m):
     inst = synth.kernel_instance(n, m)
-    _same(ob.port_dual(variant, inst), ob.ref_dual(variant, inst))
     rng = np.random.default_rng(n + 31 * m)
-    for _ in range(3):                       # other multipliers, including zeros and huge ones
-        y = rng.choice([0.0, 1e-3, 1.0, 50.0, 1e40], size=m) * rng.random(m)
-        _same(ob.port_dual(variant, inst, y), ob.ref_dual(variant, inst, y))
+    # the instance's own multipliers, then others, including zeros and huge ones
+    ys = [None] + [rng.choice([0.0, 1e-3, 1.0, 50.0, 1e40], size=m) * rng.random(m) for _ in range(3)]
+    for i, y in enumerate(ys):
+        want = reference(f"oracle_port/dual/{variant}/n={n}/m={m}/y{i}", lambda lib: _digest(ob.ref_dual(variant, inst, y)))
+        _same(_digest(ob.port_dual(variant, inst, y)), want)
 
 
-def test_port_dual_nan_constraint_switches_off_mma(built):
+def test_port_dual_nan_constraint_switches_off_mma(built, reference):
     """mma.c:78,103,126: a NaN constraint value removes that constraint from the MMA dual."""
     inst = synth.kernel_instance(5000, 3)
     inst["c0"] = np.array([-0.1, np.nan, 0.2])
     a = ob.port_dual(ob.MMA, inst)
-    if ob.ref_dual_available():
-        _same(a, ob.ref_dual(ob.MMA, inst))
+    _same(_digest(a), reference("oracle_port/dual_nan_constraint", lambda lib: _digest(ob.ref_dual(ob.MMA, inst))))
     drop = dict(inst, m=2, grad_c=inst["grad_c"][[0, 2]], c0=inst["c0"][[0, 2]], rhoc=inst["rhoc"][[0, 2]],
                 y=inst["y"][[0, 2]])
     b = ob.port_dual(ob.MMA, drop)
@@ -125,36 +135,38 @@ def _run_lib(lib, alg, n, f, cons, tols, lb, ub, x0, **kw):
         else:
             o.set_param(k, v)
     x = o.optimize(x0)
-    return dict(ret=o.last_optimize_result(), x=x, minf=o.last_optimum_value(), numevals=o.get_numevals())
+    return dict(ret=o.last_optimize_result(), x_sha256=_sha256(x), minf=o.last_optimum_value(), numevals=o.get_numevals())
 
 
 @pytest.mark.parametrize("variant", [ob.MMA, ob.CCSAQ])
-def test_port_solver_bitwise_vs_reference_rosenbrock(built, reflib, variant):
+def test_port_solver_bitwise_vs_reference_rosenbrock(built, reference, variant):
     """chained Rosenbrock + 4 dense linear constraints (the BASELINE config-3 instance, small n)."""
     import nlopt_b200 as nl
     n, m = 500, 4
     cons = [P.lin_constraint(k, n) for k in range(m)]
     lb, ub = np.full(n, -2.0), np.full(n, 2.0)
     alg = nl.LD_MMA if variant == ob.MMA else nl.LD_CCSAQ
+    b = reference(f"oracle_port/solver_rosenbrock/{variant}",
+                  lambda lib: _run_lib(lib, alg, n, P.rosen_f, cons, [1e-8] * m, lb, ub, P.rosen_x0(n), maxeval=25))
     a = ob.port_minimize(variant, P.rosen_f, cons, [1e-8] * m, lb, ub, P.rosen_x0(n), maxeval=25)
-    b = _run_lib(reflib, alg, n, P.rosen_f, cons, [1e-8] * m, lb, ub, P.rosen_x0(n), maxeval=25)
     assert a["ret"] == b["ret"] and a["numevals"] == b["numevals"]
-    assert a["minf"] == b["minf"] and np.array_equal(a["x"], b["x"])
+    assert a["minf"] == b["minf"] and _sha256(a["x"]) == b["x_sha256"]
 
 
 @pytest.mark.parametrize("variant", [ob.MMA, ob.CCSAQ])
 @pytest.mark.parametrize("x0v", [-0.5, 0.5])
-def test_port_solver_bitwise_vs_reference_quadratic(built, reflib, variant, x0v):
+def test_port_solver_bitwise_vs_reference_quadratic(built, reference, variant, x0v):
     """separable quadratic + mean constraint (config-2 shape); x0=+0.5 starts infeasible (dual_ub = 1e40 path)."""
     import nlopt_b200 as nl
     n = 2000
     f, c = P.quad_problem(n)
     lb, ub = np.full(n, -1.0), np.full(n, 1.0)
     alg = nl.LD_MMA if variant == ob.MMA else nl.LD_CCSAQ
+    b = reference(f"oracle_port/solver_quadratic/{variant}/x0={x0v}",
+                  lambda lib: _run_lib(lib, alg, n, f, [c], [0.0], lb, ub, np.full(n, x0v), xtol_rel=1e-6, maxeval=200))
     a = ob.port_minimize(variant, f, [c], [0.0], lb, ub, np.full(n, x0v), xtol_rel=1e-6, maxeval=200)
-    b = _run_lib(reflib, alg, n, f, [c], [0.0], lb, ub, np.full(n, x0v), xtol_rel=1e-6, maxeval=200)
     assert a["ret"] == b["ret"] and a["numevals"] == b["numevals"]
-    assert a["minf"] == b["minf"] and np.array_equal(a["x"], b["x"])
+    assert a["minf"] == b["minf"] and _sha256(a["x"]) == b["x_sha256"]
 
 
 def test_port_sigma_and_stop_helpers(built):
